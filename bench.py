@@ -14,6 +14,10 @@ statistics accumulated on-chip and -- at N > 1 -- all-reduced over NCCL.  Weak s
 `value` is timed with CUDA events on the launching stream with every input resident in HBM; `e2e` is the
 same metric through the C ABI with HOST buffers (pinned), the host->device copies of the scenario and the
 device->host read of the statistics inside the timed region.
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (float64): the all-reduced
+statistics and the state and covariance of a fixed sample of this rank's filters.  The inputs depend on the
+arguments only, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -30,6 +34,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from
 
 # Floating-point operations executed per call by the structured code (FMA = 2), measured with an
 # instrumented scalar type (tests/host_core hc_count_flops; tests/test_flop_count.py pins these numbers).
@@ -39,6 +44,8 @@ JOSEPH_EXTRA_FLOPS = {1: 2 * 2 * 36 * 15, 0: 2 * 2 * 36 * 9}
 # Algorithmic HBM bytes per filter-step in Monte-Carlo mode: state + covariance load and store
 # (16 + 120 doubles each way) amortised over the ticks of one launch; the shared clean scenario is L2-resident.
 STATE_BYTES = (16 + 120) * 8 * 2
+# --dump-outputs: filters whose state and covariance are written (a seeded sample when the rank owns more); 7.6 MB in all
+DUMP_FILTERS, DUMP_SEED = 4096, 20240
 
 
 def bench_params(q, multirate=False, dynamic=False):
@@ -375,6 +382,16 @@ class Leg:
                 "tolerance": 1e-9 if self.prec == self.q.QEKF_FP64 else 1e-4,
                 "against": "oracle/ekf_oracle.c replaying the device's dumped noise realisation (FP64)"}
 
+    def outputs(self):
+        """What the last pass left for its caller: the all-reduced statistics and the state / covariance of up to
+        DUMP_FILTERS of this rank's filters (local ids drawn with a fixed seed), all float64."""
+        b, N = self.b, self.N
+        self.torch.cuda.synchronize()
+        ids = np.arange(N) if N <= DUMP_FILTERS else np.sort(np.random.default_rng(DUMP_SEED).choice(N, DUMP_FILTERS, replace=False))
+        return {"stats": self.stats_dev.cpu().numpy(), "filter_ids": ids.astype(np.float64),
+                "state": np.concatenate([b.state(int(i), 1) for i in ids], axis=1),
+                "cov": np.concatenate([b.cov(int(i), 1) for i in ids], axis=2)}
+
     def close(self):
         self.b.close()
         self._keep = None
@@ -448,6 +465,10 @@ def run_ours(args):
     ms_total = main.timed(main.sh, False, args.steps, dist)
     launches = b.launch_count - l0
     n_pred, n_corr = b.step_counts(reset=True)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in main.outputs().items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     k_ms = main.kernel_ms(2)
     clocks = sampler.stop()
     main.one_step(hs, True)                              # warm the host path (staging slab allocation)
@@ -611,7 +632,14 @@ def main():
                     help="weak: --filters per GPU (default); strong: --filters in total, split over the ranks")
     ap.add_argument("--no-stats", action="store_true", help="diagnostic: never sample statistics")
     ap.add_argument("--no-private-dropout", action="store_true", help="diagnostic: drop the per-filter dropout window")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy: statistics, filter_ids and the "
+                         "state / covariance of those filters (rank 0's)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

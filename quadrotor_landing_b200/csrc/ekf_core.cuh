@@ -80,11 +80,12 @@ template <typename T> struct Consts {
     T r_v_cv[3];
     T q_vc[4];            // normalised + clipped, xyzw                   (cpp:121)
     T cov_init[5];        // r, v, ang, ab, wb                            (cpp:102-113)
-    T Kcam[6];            // camera_K rows 0 and 1
-    T u_lo, u_hi, v_lo, v_hi; // width*margin, width*(1-margin), height*margin, height*(1-margin)  (cpp:176-179)
-    T cam_w, cam_h;           // camera_width, camera_height
-    T tag_hw[16];         // tag_widths/2
-    T tag_px[16], tag_py[16];
+    // camera and bundle geometry in double whatever T: the corner-margin gate is evaluated in double (corner_gate)
+    double Kcam[6];       // camera_K rows 0 and 1
+    double u_lo, u_hi, v_lo, v_hi; // width*margin, width*(1-margin), height*margin, height*(1-margin)  (cpp:176-179)
+    double cam_w, cam_h;      // camera_width, camera_height
+    double tag_hw[16];    // tag_widths/2
+    double tag_px[16], tag_py[16];
     T small_ang_tol;
     double meas_delay, meas_delay_max, dyn_offset;   // seconds; the delay -> step rounding is done in double (cpp:199-200)
     double dT_nom;        // 1/update_freq in double, for the same reason
@@ -844,6 +845,31 @@ template <typename T> QEKF_FN void refine_gain_row(const T b[6], const T S[21], 
     }
 }
 
+// x + a[0] g[0] + a[sa] g[1] + a[2 sa] g[2] in double, returned as hi + lo in T: the conventional model's columns of
+// B = P G^T (G = [I Gam; 0 I]) carried to about u^2 in the FP32 mode (see correction_step)
+template <typename T> QEKF_FN T gam_dot(T x, const T *a, int sa, const T g[3], T &lo)
+{
+    double v = (double)x;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) v = M<double>::fma_((double)a[k * sa], (double)g[k], v);
+    const T hi = (T)v;
+    lo = (T)(v - (double)hi);
+    return hi;
+}
+
+// one gain row from the compensated B row in double: k = (b + blo) S^-1, blo covering columns 0..2
+template <typename T> QEKF_FN void gain_row_f64(const T b[6], const T blo[3], const double Sinv[21], T k[6])
+{
+#pragma unroll
+    for (int m = 0; m < 6; ++m) {
+        double v = 0.0;
+#pragma unroll
+        for (int l = 0; l < 6; ++l)
+            v = M<double>::fma_((double)b[l] + (l < 3 ? (double)blo[l] : 0.0), Sinv[sym_idx<6>(l, m)], v);
+        k[m] = (T)v;
+    }
+}
+
 // outputs of a correction that the reference keeps as members (cpp:431,438,443)
 template <typename T> struct Observation {
     T r_t_vt_obs[3];
@@ -858,6 +884,13 @@ template <typename T> struct Observation {
 //     K_X = B_X S^-1,   P^_XY = P_XY - K_X B_Y^T,   dx_X = K_X dy,
 // i.e. exactly  P^ = (I - K G) P  and  dx = K dy  without materialising K or I - K G.
 // JOSEPH selects the symmetrised Joseph form used by the FP32 mode.
+// The refined gain leaves an error of order (kappa(S) u)^2 in the covariance.  For the direct model S = P_obs + R_k and
+// kappa(S) stays ~1e3 even for stiff updates; for the conventional model G mixes position and attitude through
+// Gam = C skew(C^T r) and kappa(S) reaches ~1e5, where that error exceeds the smallest posterior eigenvalues of stiff
+// updates (condition ~1e7) and the covariance came out indefinite.  So in the FP32 mode the conventional model (CB
+// below) forms B's columns 0..2 = P_.r + P_.th Gam^T in double and keeps them as hi + lo, forms and inverts S in double,
+// computes the gain rows in double (accurate to ~u, no refinement needed) and subtracts K (hi + lo)^T.  Once per
+// correction; the FP64 path and the direct model are unchanged.
 // ------------------------------------------------------------------------------------------------
 // The measurement-model part of correction_step (cpp:417-472): observed pose, innovation dy, R_k = N R N^T
 // (packed upper 6x6) and, for the conventional model, Gam = C skew(C^T r).  Needs the nominal attitude and
@@ -954,10 +987,13 @@ template <typename T, bool BIAS, bool DIRECT, class PS, class PAR>
 QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &par, Observation<T> &obs)
 {
     constexpr int NB = BIAS ? 5 : 3;
+    constexpr bool CB = UpdateForm<T>::joseph && !DIRECT;     // compensated B (see above)
     T dy[6];
     T Sinv[21];
     T S[21];         // innovation covariance G P G^T + R_k, packed upper triangle
     T Brt[36];       // rows: dr(0..2), dtheta(3..5) of  P_[r,th],. G^T   (6x6)
+    T BrtLo[18];     // CB: low parts of Brt's columns 0..2, [row][3]
+    double SinvD[CB ? 21 : 1];   // CB: S^-1 in double
     T Gam[9];
     {
         T Rk[21];
@@ -977,7 +1013,32 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
                     Brt[(3 + a) * 6 + b] = rt[b * 3 + a];
                     Brt[(3 + a) * 6 + 3 + b] = tt[a * 3 + b];
                 }
-            if (!DIRECT) {
+            if (CB) {
+                // columns 0..2 += (.,th) Gam^T in double, kept as hi + lo; S = G B + R_k and S^-1 from them in double
+                double Sd[21];
+#pragma unroll
+                for (int a = 0; a < 3; ++a)
+#pragma unroll
+                    for (int b = 0; b < 3; ++b) {
+                        Brt[a * 6 + b] = gam_dot(Brt[a * 6 + b], rt + a * 3, 1, Gam + b * 3, BrtLo[a * 3 + b]);
+                        Brt[(3 + a) * 6 + b] = gam_dot(Brt[(3 + a) * 6 + b], tt + a * 3, 1, Gam + b * 3, BrtLo[(3 + a) * 3 + b]);
+                    }
+#pragma unroll
+                for (int i = 0; i < 6; ++i)
+#pragma unroll
+                    for (int j = i; j < 6; ++j) {
+                        double x = (double)Brt[i * 6 + j] + (j < 3 ? (double)BrtLo[i * 3 + j] : 0.0);
+                        if (i < 3) {
+#pragma unroll
+                            for (int k = 0; k < 3; ++k) {
+                                const double bkj = (double)Brt[(3 + k) * 6 + j] + (j < 3 ? (double)BrtLo[(3 + k) * 3 + j] : 0.0);
+                                x = M<double>::fma_((double)Gam[i * 3 + k], bkj, x);
+                            }
+                        }
+                        Sd[sym_idx<6>(i, j)] = x + (double)Rk[sym_idx<6>(i, j)];
+                    }
+                sym6_inverse(Sd, SinvD);
+            } else if (!DIRECT) {
                 // columns 0..2 += (.,th) Gam^T
 #pragma unroll
                 for (int a = 0; a < 3; ++a)
@@ -1010,7 +1071,7 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
 #pragma unroll
                     for (int j = i; j < 6; ++j) S[sym_idx<6>(i, j)] = Brt[i * 6 + j] + Rk[sym_idx<6>(i, j)];
             }
-            sym6_inverse(S, Sinv);
+            if (!CB) sym6_inverse(S, Sinv);
         }
     }
 
@@ -1019,7 +1080,7 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
 #pragma unroll
     for (int xi = 0; xi < NB - 2; ++xi) {
         const int X = (xi == 0) ? BV : (xi == 1 ? BAB : BWB);
-        T Bx[18], Kx[18];
+        T Bx[18], Kx[18], BxLo[9];
         {
             T xr[9], xt[9];
             ldb(P, X, BR, xr);
@@ -1029,7 +1090,9 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
 #pragma unroll
                 for (int b = 0; b < 3; ++b) {
                     T x0 = xr[a * 3 + b];
-                    if (!DIRECT) {
+                    if (CB) {
+                        x0 = gam_dot(x0, xt + a * 3, 1, Gam + b * 3, BxLo[a * 3 + b]);
+                    } else if (!DIRECT) {
 #pragma unroll
                         for (int k = 0; k < 3; ++k) x0 = M<T>::fma_(xt[a * 3 + k], Gam[b * 3 + k], x0);
                     }
@@ -1039,6 +1102,10 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
         }
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
+            if (CB) {
+                gain_row_f64(Bx + a * 6, BxLo + a * 3, SinvD, Kx + a * 6);
+                continue;
+            }
 #pragma unroll
             for (int m = 0; m < 6; ++m) {
                 T v = T(0);
@@ -1066,10 +1133,14 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
 #pragma unroll
         for (int yi = xi; yi < NB - 2; ++yi) {
             const int Y = (yi == 0) ? BV : (yi == 1 ? BAB : BWB);
-            T By[18];
+            T By[18], ByLo[9];
             if (yi == xi) {
 #pragma unroll
                 for (int i = 0; i < 18; ++i) By[i] = Bx[i];
+                if (CB) {
+#pragma unroll
+                    for (int i = 0; i < 9; ++i) ByLo[i] = BxLo[i];
+                }
             } else {
                 T yr[9], yt[9];
                 ldb(P, Y, BR, yr);
@@ -1079,7 +1150,9 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
 #pragma unroll
                     for (int b = 0; b < 3; ++b) {
                         T x0 = yr[a * 3 + b];
-                        if (!DIRECT) {
+                        if (CB) {
+                            x0 = gam_dot(x0, yt + a * 3, 1, Gam + b * 3, ByLo[a * 3 + b]);
+                        } else if (!DIRECT) {
 #pragma unroll
                             for (int k = 0; k < 3; ++k) x0 = M<T>::fma_(yt[a * 3 + k], Gam[b * 3 + k], x0);
                         }
@@ -1095,6 +1168,10 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
                     T v = P.ld(3 * X + a, 3 * Y + b);
 #pragma unroll
                     for (int m = 0; m < 6; ++m) v = M<T>::fma_(-Kx[a * 6 + m], By[b * 6 + m], v);
+                    if (CB) {
+#pragma unroll
+                        for (int m = 0; m < 3; ++m) v = M<T>::fma_(-Kx[a * 6 + m], ByLo[b * 3 + m], v);
+                    }
                     P.st(3 * X + a, 3 * Y + b, v);
                 }
         }
@@ -1110,6 +1187,13 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
                     v0 = M<T>::fma_(-Kx[a * 6 + m], Brt[b * 6 + m], v0);
                     v1 = M<T>::fma_(-Kx[a * 6 + m], Brt[(3 + b) * 6 + m], v1);
                 }
+                if (CB) {
+#pragma unroll
+                    for (int m = 0; m < 3; ++m) {
+                        v0 = M<T>::fma_(-Kx[a * 6 + m], BrtLo[b * 3 + m], v0);
+                        v1 = M<T>::fma_(-Kx[a * 6 + m], BrtLo[(3 + b) * 3 + m], v1);
+                    }
+                }
                 P.st(3 * BR + b, 3 * X + a, v0);
                 if (X == BV) P.st(3 * X + a, 3 * BTH + b, v1);
                 else P.st(3 * BTH + b, 3 * X + a, v1);
@@ -1119,14 +1203,18 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
 #pragma unroll
     for (int i = 0; i < 6; ++i) {
         T k[6];
+        if (CB) {
+            gain_row_f64(Brt + i * 6, BrtLo + i * 3, SinvD, k);
+        } else {
 #pragma unroll
-        for (int m = 0; m < 6; ++m) {
-            T v = T(0);
+            for (int m = 0; m < 6; ++m) {
+                T v = T(0);
 #pragma unroll
-            for (int l = 0; l < 6; ++l) v = M<T>::fma_(Brt[i * 6 + l], Sinv[sym_idx<6>(l, m)], v);
-            k[m] = v;
+                for (int l = 0; l < 6; ++l) v = M<T>::fma_(Brt[i * 6 + l], Sinv[sym_idx<6>(l, m)], v);
+                k[m] = v;
+            }
+            if (UpdateForm<T>::joseph) refine_gain_row(Brt + i * 6, S, Sinv, k);
         }
-        if (UpdateForm<T>::joseph) refine_gain_row(Brt + i * 6, S, Sinv, k);
         T dx = T(0);
 #pragma unroll
         for (int m = 0; m < 6; ++m) dx = M<T>::fma_(k[m], dy[m], dx);
@@ -1139,6 +1227,10 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
             T v = P.ld(gi, gj);
 #pragma unroll
             for (int m = 0; m < 6; ++m) v = M<T>::fma_(-k[m], Brt[j * 6 + m], v);
+            if (CB) {
+#pragma unroll
+                for (int m = 0; m < 3; ++m) v = M<T>::fma_(-k[m], BrtLo[j * 3 + m], v);
+            }
             P.st(gi, gj, v);
         }
     }
@@ -1160,25 +1252,28 @@ QEKF_FN void correction_step(Nominal<T> &s, PS &P, const T tag[7], const PAR &pa
 // ------------------------------------------------------------------------------------------------
 // corner-margin gate                                            relative_pose_EKF.cpp:156-186
 // ------------------------------------------------------------------------------------------------
-template <typename T> QEKF_FN bool corner_gate(const T tag[7], const Consts<T> &c)
+// Evaluated in double on the double tag pose whatever the filter's type T: the decision is discrete, and in float the
+// rounding of the projection (~1e-4 px at 752 px) would flip the poses whose extreme corner lies that close to a
+// margin line.  Once per arrival, so the FP32 mode pays nothing for it; in FP64 it is the same arithmetic as before.
+template <typename T> QEKF_FN bool corner_gate(const double tag[7], const Consts<T> &c)
 {
-    T Rct[9];
+    double Rct[9];
     quat_to_rot(tag + 3, Rct);
     bool ok = false;
     for (int i = 0; i < c.n_tags; ++i) {
-        const T hw = c.tag_hw[i], px0 = c.tag_px[i], py0 = c.tag_py[i];
-        T min_u = T(0), max_u = T(0), min_v = T(0), max_v = T(0);
+        const double hw = c.tag_hw[i], px0 = c.tag_px[i], py0 = c.tag_py[i];
+        double min_u = 0.0, max_u = 0.0, min_v = 0.0, max_v = 0.0;
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-            const T cx = ((k == 0 || k == 3) ? hw : -hw) + px0;
-            const T cy = ((k < 2) ? hw : -hw) + py0;
-            T pc0 = Rct[0] * cx + Rct[1] * cy + tag[0];
-            T pc1 = Rct[3] * cx + Rct[4] * cy + tag[1];
-            T pc2 = Rct[6] * cx + Rct[7] * cy + tag[2];
-            T iz = T(1) / pc2;
-            T xn = pc0 * iz, yn = pc1 * iz, zn = pc2 * iz;
-            T uu = c.Kcam[0] * xn + c.Kcam[1] * yn + c.Kcam[2] * zn;
-            T vv = c.Kcam[3] * xn + c.Kcam[4] * yn + c.Kcam[5] * zn;
+            const double cx = ((k == 0 || k == 3) ? hw : -hw) + px0;
+            const double cy = ((k < 2) ? hw : -hw) + py0;
+            double pc0 = Rct[0] * cx + Rct[1] * cy + tag[0];
+            double pc1 = Rct[3] * cx + Rct[4] * cy + tag[1];
+            double pc2 = Rct[6] * cx + Rct[7] * cy + tag[2];
+            double iz = 1.0 / pc2;
+            double xn = pc0 * iz, yn = pc1 * iz, zn = pc2 * iz;
+            double uu = c.Kcam[0] * xn + c.Kcam[1] * yn + c.Kcam[2] * zn;
+            double vv = c.Kcam[3] * xn + c.Kcam[4] * yn + c.Kcam[5] * zn;
             if (k == 0) { min_u = max_u = uu; min_v = max_v = vv; }
             else {
                 min_u = uu < min_u ? uu : min_u; max_u = uu > max_u ? uu : max_u;

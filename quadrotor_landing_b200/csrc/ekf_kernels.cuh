@@ -620,14 +620,17 @@ QEKF_FN void run_filter(const RunArgs<T> &a, const int64_t i_in, PS &P, int32_t 
         if (want && serve) {
             // ---- consume the measurement, corner-margin gate (cpp:150-186), single-rate correction (cpp:265-279) ----
             T tag[7];
+            double tg[7];       // the gate decides on the double pose
             if (pend_m >= 0) {
-                in.tag(a.in, a.ns, pend_m, tag);
+                in.tag_f64(a.in, a.ns, pend_m, tg);
             } else {
 #pragma unroll
-                for (int cc = 0; cc < 7; ++cc) tag[cc] = (T)a.st.pend[cc * a.st.ld + i];
+                for (int cc = 0; cc < 7; ++cc) tg[cc] = a.st.pend[cc * a.st.ld + i];
             }
+#pragma unroll
+            for (int cc = 0; cc < 7; ++cc) tag[cc] = (T)tg[cc];
             flags &= ~FLAG_READY;
-            const bool perform = c.corner_margin_enbl ? corner_gate<T>(tag, c) : true;
+            const bool perform = c.corner_margin_enbl ? corner_gate<T>(tg, c) : true;
             held = 0;
             if (perform) {
                 ++n_corr;
@@ -868,16 +871,19 @@ QEKF_FN void run_filter_mr(const RunArgs<T> &a, const int64_t i_in, PS &P, int32
         T tag[7];
         double stamp = 0;
         if (exec && want) {
+            double tg[7];       // the gate decides on the double pose
             if (pend_m >= 0) {
-                in.tag(a.in, a.ns, pend_m, tag);
+                in.tag_f64(a.in, a.ns, pend_m, tg);
                 stamp = a.in.tag_stamp[pend_m];
             } else {
 #pragma unroll
-                for (int cc = 0; cc < 7; ++cc) tag[cc] = (T)a.st.pend[cc * a.st.ld + i];
+                for (int cc = 0; cc < 7; ++cc) tg[cc] = a.st.pend[cc * a.st.ld + i];
                 stamp = a.st.pend[7 * a.st.ld + i];
             }
+#pragma unroll
+            for (int cc = 0; cc < 7; ++cc) tag[cc] = (T)tg[cc];
             flags &= ~FLAG_READY;
-            perform = c.corner_margin_enbl ? corner_gate<T>(tag, c) : true;
+            perform = c.corner_margin_enbl ? corner_gate<T>(tg, c) : true;
             held = 0;
         }
 
@@ -1160,16 +1166,19 @@ QEKF_FN void run_filter_mrs(const RunArgs<T> &a, const int64_t i_in, PS &P, int3
         T tag[7];
         double stamp = 0;
         if (exec) {
+            double tg[7];       // the gate decides on the double pose
             if (pend_m >= 0) {
-                in.tag(a.in, a.ns, pend_m, tag);
+                in.tag_f64(a.in, a.ns, pend_m, tg);
                 stamp = a.in.tag_stamp[pend_m];
             } else {
 #pragma unroll
-                for (int cc = 0; cc < 7; ++cc) tag[cc] = (T)a.st.pend[cc * a.st.ld + i];
+                for (int cc = 0; cc < 7; ++cc) tg[cc] = a.st.pend[cc * a.st.ld + i];
                 stamp = a.st.pend[7 * a.st.ld + i];
             }
+#pragma unroll
+            for (int cc = 0; cc < 7; ++cc) tag[cc] = (T)tg[cc];
             flags &= ~FLAG_READY;
-            perform = c.corner_margin_enbl ? corner_gate<T>(tag, c) : true;
+            perform = c.corner_margin_enbl ? corner_gate<T>(tg, c) : true;
             held = 0;
         }
         // ---- how far this lane moves its checkpoint now ----

@@ -64,18 +64,18 @@ template <typename T> Consts<T> make_consts(const qekf_params &p)
         for (int j = 0; j < 3; ++j) c.D[k * 3 + j] = (T)(p.R_ang[k] * C[j * 3 + k]);
     c.cov_init[0] = (T)p.r_cov_init; c.cov_init[1] = (T)p.v_cov_init; c.cov_init[2] = (T)p.ang_cov_init;
     c.cov_init[3] = (T)p.ab_cov_init; c.cov_init[4] = (T)p.wb_cov_init;
-    for (int i = 0; i < 6; ++i) c.Kcam[i] = (T)p.camera_K[i];
-    c.u_lo = (T)(p.camera_width * p.tag_in_view_margin);
-    c.u_hi = (T)(p.camera_width * (1 - p.tag_in_view_margin));
-    c.v_lo = (T)(p.camera_height * p.tag_in_view_margin);
-    c.v_hi = (T)(p.camera_height * (1 - p.tag_in_view_margin));
-    c.cam_w = (T)p.camera_width;
-    c.cam_h = (T)p.camera_height;
+    for (int i = 0; i < 6; ++i) c.Kcam[i] = p.camera_K[i];
+    c.u_lo = p.camera_width * p.tag_in_view_margin;
+    c.u_hi = p.camera_width * (1 - p.tag_in_view_margin);
+    c.v_lo = p.camera_height * p.tag_in_view_margin;
+    c.v_hi = p.camera_height * (1 - p.tag_in_view_margin);
+    c.cam_w = p.camera_width;
+    c.cam_h = p.camera_height;
     c.n_tags = p.n_tags;
     for (int i = 0; i < QEKF_MAX_TAGS; ++i) {
-        c.tag_hw[i] = (T)(p.tag_widths[i] / 2);
-        c.tag_px[i] = (T)p.tag_positions[3 * i + 0];
-        c.tag_py[i] = (T)p.tag_positions[3 * i + 1];
+        c.tag_hw[i] = p.tag_widths[i] / 2;
+        c.tag_px[i] = p.tag_positions[3 * i + 0];
+        c.tag_py[i] = p.tag_positions[3 * i + 1];
     }
     c.small_ang_tol = (T)p.small_ang_tol;
     c.meas_delay = p.measurement_delay;

@@ -121,7 +121,7 @@ template <typename T> struct RunArgs {
     int64_t k0, n_steps;
     int32_t m0;           // first arrival with tag_step >= k0
     NoiseSpec ns;         // SYNTH launches only
-    StatsView stats;      // SYNTH launches only (acc == nullptr: no statistics)
+    StatsView stats;      // acc == nullptr: no statistics
 };
 
 #ifdef __CUDA_ARCH__
@@ -219,13 +219,15 @@ template <typename T, bool SYNTH> struct Inputs {
     }
 };
 
-// One statistics sample after tick k (SYNTH launches: the truth and the true bias are known).  Called by every
+// One statistics sample after tick k.  Where the truth comes from is decided at compile time: SYNTH (Monte-Carlo)
+// launches read the shared scenario truth and get the filter's true bias from the caller; explicit-stream launches
+// read row i of the per-filter truth, bin by bin, true bias included (StatsView::truth_pf).  Called by every
 // lane of the CTA at the same point (`valid` = this lane holds an initialised filter that is at the sampling
 // tick), so that the 20 sums can be reduced over the warp with shuffles and leave as ONE atomic per warp and
 // statistic instead of one per lane.  Deliberately NOT inlined on the device: it runs once per `stride` ticks
 // and must not take part in the register allocation of the hot loop.
 // (SAVE is a leftover of the in-place NEES factorisation, which had to park P in HBM; the covariance is only read now.)
-template <typename T, bool BIAS, class PS, bool SAVE = true>
+template <typename T, bool BIAS, class PS, bool SAVE = true, bool SYNTH = true>
 QEKF_COLD void stats_sample(const RunArgs<T> &a, int64_t i, int64_t k, const Nominal<T> s, PS P, const double *bias,
                             bool valid)
 {
@@ -240,19 +242,23 @@ QEKF_COLD void stats_sample(const RunArgs<T> &a, int64_t i, int64_t k, const Nom
 #pragma unroll
     for (int c = 0; c < STAT_DIM; ++c) sum[c] = 0.0;
     if (valid) {
-        const double *tr = sv.truth + (k + 1) * 10;
+        // component c of the true state (r v q_tv ab wb); the bias components only exist per filter
+        auto tr = [&](int c) -> double {
+            return SYNTH ? sv.truth[(k + 1) * 10 + c] : sv.truth_pf[((int64_t)bin * 16 + c) * sv.ld_t + i];
+        };
         T e[N];
 #pragma unroll
-        for (int c = 0; c < 3; ++c) { e[c] = (T)tr[c] - s.r[c]; e[3 + c] = (T)tr[3 + c] - s.v[c]; }
+        for (int c = 0; c < 3; ++c) { e[c] = (T)tr(c) - s.r[c]; e[3 + c] = (T)tr(3 + c) - s.v[c]; }
         {
-            T qt[4] = { (T)tr[6], (T)tr[7], (T)tr[8], (T)tr[9] }, dq[4];
+            T qt[4] = { (T)tr(6), (T)tr(7), (T)tr(8), (T)tr(9) }, dq[4];
             quat_conj_mul(s.q, qt, dq);
             quat_normclip(dq);
             quat_log(dq, e + 6);
         }
         if (BIAS) {
+            auto tb = [&](int c) -> double { return SYNTH ? bias[c] : tr(10 + c); };
 #pragma unroll
-            for (int c = 0; c < 3; ++c) { e[9 + c] = (T)bias[c] - s.ab[c]; e[12 + c] = (T)bias[3 + c] - s.wb[c]; }
+            for (int c = 0; c < 3; ++c) { e[9 + c] = (T)tb(c) - s.ab[c]; e[12 + c] = (T)tb(3 + c) - s.wb[c]; }
         }
         // (the covariance is only read: see nees_readonly)
         T nees;
@@ -476,7 +482,11 @@ constexpr int SR_SCRATCH_INTS = 16;
 // Statistics fence: a lane that has finished a sampling tick waits until every lane of the CTA has, then all
 // sample together (one execution of the sampling code per stride; the time skew is back to zero).
 // `live` = false marks the padding lanes of a ragged last CTA (they only take part in the votes).
-template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool PF, class PS, bool CSM = false>
+// STATS: the fence and the sampling are compiled in (Monte-Carlo launches, and explicit-stream launches scored against
+// per-filter truth).  The unscored explicit kernels leave them out: compiled in, with the statistics switched off at
+// run time, they cost those kernels 1.0 % (FP64, N = 65,536) and 2.4 % (FP64 conventional model, N = 1M) in
+// tools/perf_probe.py on a B200.
+template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool PF, class PS, bool CSM = false, bool STATS = SYNTH>
 QEKF_FN void run_filter(const RunArgs<T> &a, const int64_t i_in, PS &P, int32_t *scr, const int scr_stride,
                         const bool live = true, int *vbuf = nullptr, const Consts<T> *c_cold = nullptr)
 {
@@ -525,7 +535,7 @@ QEKF_FN void run_filter(const RunArgs<T> &a, const int64_t i_in, PS &P, int32_t 
     pend_m = -1;                       // index of the latched arrival; -1 = latched pose lives in st.pend
     held = 0;                          // iterations this lane has held its correction back
     bool at_fence = false;             // finished a sampling tick; waiting for the CTA to catch up
-    const bool do_stats = SYNTH && a.stats.acc != nullptr;
+    const bool do_stats = STATS && a.stats.acc != nullptr;
     const int32_t patience = c.limit_measurement_freq ? (c.upd_per_meas - 1) : 0;
     // the next sampling boundary (a multiple of the stride): every lane of the CTA stops there until all have arrived, so
     // it is the same for all of them and moves on when the sample is taken -- no k % stride on the per-tick path
@@ -603,7 +613,7 @@ QEKF_FN void run_filter(const RunArgs<T> &a, const int64_t i_in, PS &P, int32_t 
             const bool mine = live && at_fence && (fl0 & FLAG_INIT);
             double tb[6] = { 0, 0, 0, 0, 0, 0 };
             if (SYNTH) true_bias_now(tb);
-            stats_sample<T, BIAS>(a, i, (int64_t)k - 1, s, P, tb, mine);
+            stats_sample<T, BIAS, PS, true, SYNTH>(a, i, (int64_t)k - 1, s, P, tb, mine);
             if (mine) ++n_sexec;
             at_fence = false;
             next_fence += a.stats.stride;
@@ -759,7 +769,7 @@ QEKF_COLD void advance_call(Nominal<T> *sp, PS &P, const PAR par, const T *ring_
 // step delay), so every index a future correction can address is still reachable.  Lanes that do not correct
 // (tag dropout, rejected detection) catch their checkpoint up to size-D inside their CTA-mates' correction
 // events, where the warp executes prediction code anyway.
-template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool PF, class PS, bool CSM = false>
+template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool PF, class PS, bool CSM = false, bool STATS = SYNTH>
 QEKF_FN void run_filter_mr(const RunArgs<T> &a, const int64_t i_in, PS &P, int32_t *scr, const int scr_stride,
                            const bool live = true, int *vbuf = nullptr, const Consts<T> *c_cold = nullptr)
 {
@@ -809,7 +819,7 @@ QEKF_FN void run_filter_mr(const RunArgs<T> &a, const int64_t i_in, PS &P, int32
     pend_m = -1;
     held = 0;
     bool at_fence = false;
-    const bool do_stats = SYNTH && a.stats.acc != nullptr;
+    const bool do_stats = STATS && a.stats.acc != nullptr;          // see run_filter
     const int32_t patience = c.limit_measurement_freq ? (c.upd_per_meas - 1) : 0;
     int32_t next_fence = do_stats ? (int32_t)((a.k0 / a.stats.stride + 1) * a.stats.stride) : INT32_MAX;   // see run_filter
 
@@ -852,7 +862,7 @@ QEKF_FN void run_filter_mr(const RunArgs<T> &a, const int64_t i_in, PS &P, int32
             }
             double tb[6] = { 0, 0, 0, 0, 0, 0 };
             if (SYNTH) true_bias_now(tb);
-            stats_sample<T, BIAS>(a, i, k - 1, head, P, tb, mine);
+            stats_sample<T, BIAS, PS, true, SYNTH>(a, i, k - 1, head, P, tb, mine);
             if (mine) {
                 load_checkpoint<T>(a.st, i, s, P);
                 ++n_sexec;
@@ -1300,8 +1310,8 @@ template <typename T> __device__ __forceinline__ void copy_consts(Consts<T> *dst
 }
 constexpr size_t consts_smem_bytes(size_t consts_size) { return (consts_size + 15) / 16 * 16; }
 
-// fused multi-tick replay: MR = false single-rate filter, MR = true delayed-measurement fusion
-template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool MR, bool PF, int BLOCK>
+// fused multi-tick replay: MR = false single-rate filter, MR = true delayed-measurement fusion; STATS: see run_filter
+template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool MR, bool PF, int BLOCK, bool STATS = SYNTH>
 __global__ void __launch_bounds__(BLOCK, 1) run_kernel(const __grid_constant__ RunArgs<T> a)
 {
     constexpr int N = BIAS ? 15 : 9;
@@ -1328,11 +1338,11 @@ __global__ void __launch_bounds__(BLOCK, 1) run_kernel(const __grid_constant__ R
 #ifndef QEKF_EXP8
     if constexpr (MR && SYNTH) {
         if (a.st.hist_synth) run_filter_mrs<T, BIAS, DIRECT, PF, PShared<T, N, BLOCK>, true>(a, i, P, scr + threadIdx.x, BLOCK, live, vbuf, csm);
-        else run_filter_mr<T, BIAS, DIRECT, SYNTH, PF, PShared<T, N, BLOCK>, true>(a, i, P, scr + threadIdx.x, BLOCK, live, vbuf, csm);
+        else run_filter_mr<T, BIAS, DIRECT, SYNTH, PF, PShared<T, N, BLOCK>, true, STATS>(a, i, P, scr + threadIdx.x, BLOCK, live, vbuf, csm);
     } else if constexpr (MR) {
-        run_filter_mr<T, BIAS, DIRECT, SYNTH, PF, PShared<T, N, BLOCK>, true>(a, i, P, scr + threadIdx.x, BLOCK, live, vbuf, csm);
+        run_filter_mr<T, BIAS, DIRECT, SYNTH, PF, PShared<T, N, BLOCK>, true, STATS>(a, i, P, scr + threadIdx.x, BLOCK, live, vbuf, csm);
     } else {
-        run_filter<T, BIAS, DIRECT, SYNTH, PF, PShared<T, N, BLOCK>, true>(a, i, P, scr + threadIdx.x, BLOCK, live, vbuf, csm);
+        run_filter<T, BIAS, DIRECT, SYNTH, PF, PShared<T, N, BLOCK>, true, STATS>(a, i, P, scr + threadIdx.x, BLOCK, live, vbuf, csm);
     }
 #else
     if (MR) run_filter_mr<T, BIAS, DIRECT, SYNTH, PF>(a, i, P, scr + threadIdx.x, BLOCK, live, vbuf, csm);

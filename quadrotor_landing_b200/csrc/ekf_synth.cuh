@@ -242,7 +242,11 @@ constexpr int STAT_REPL = 32;     // replicas of the accumulator (spreads atomic
 
 struct StatsView {
     double *acc;                  // [STAT_REPL][n_bins][STAT_DIM]
-    const double *truth;          // [T+1][10] r v q_tv; state after tick k is truth[k+1]
+    const double *truth;          // Monte-Carlo launches: [T+1][10] r v q_tv shared by all filters; state after tick k is truth[k+1]
+    // explicit-stream launches: each filter's own truth, element (bin b, component c) of filter row i at
+    // truth_pf[(b*16 + c)*ld_t + i], components r v q_tv ab wb (the state after the sampling tick of bin b)
+    const double *truth_pf;
+    int64_t ld_t;
     int32_t n_bins;
     int32_t stride;               // sample after tick k when (k+1) % stride == 0
     double chi2_lo, chi2_hi;

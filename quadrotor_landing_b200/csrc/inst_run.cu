@@ -5,10 +5,10 @@
 
 namespace qekf {
 
-template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool MR, bool PF>
+template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool MR, bool PF, bool STATS>
 cudaError_t launch_run(const RunArgs<T> &a, unsigned grid, size_t smem, cudaStream_t stream)
 {
-    auto kern = run_kernel<T, BIAS, DIRECT, SYNTH, MR, PF, BlockOf<T>::value>;
+    auto kern = run_kernel<T, BIAS, DIRECT, SYNTH, MR, PF, BlockOf<T>::value, STATS>;
     cudaError_t e = prep_kernel(kern, smem);
     if (e != cudaSuccess) return e;
     kern<<<grid, BlockOf<T>::value, smem, stream>>>(a);
@@ -37,12 +37,15 @@ cudaError_t launch_tick(const RunArgs<T> &a, const double *pose8, int tag_mode, 
 template cudaError_t launch_tick<Q_T, (Q_BIAS != 0), (Q_DIRECT != 0), (Q_MR != 0)>(const RunArgs<Q_T> &, const double *, int,
                                                                                    double *, int, cudaStream_t);
 
-#define INST(S, PF_)                                                                                                  \
-    template cudaError_t launch_run<Q_T, (Q_BIAS != 0), (Q_DIRECT != 0), S, (Q_MR != 0), PF_>(const RunArgs<Q_T> &,    \
-                                                                                               unsigned, size_t, cudaStream_t);
-INST(false, false)
-INST(true, false)
-INST(false, true)
-INST(true, true)
+#define INST(S, PF_, ST)                                                                                              \
+    template cudaError_t launch_run<Q_T, (Q_BIAS != 0), (Q_DIRECT != 0), S, (Q_MR != 0), PF_, ST>(const RunArgs<Q_T> &, \
+                                                                                                   unsigned, size_t,      \
+                                                                                                   cudaStream_t);
+INST(false, false, false)
+INST(true, false, true)
+INST(false, true, false)
+INST(true, true, true)
+INST(false, false, true)      // explicit streams scored against per-filter truth (qekf_run_with_truth)
+INST(false, true, true)
 
 }  // namespace qekf

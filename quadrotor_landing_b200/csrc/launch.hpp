@@ -21,7 +21,7 @@ template <typename T> struct BlockOf { static constexpr int value = (sizeof(T) =
 template <typename T> struct BlockOf { static constexpr int value = (sizeof(T) == 4) ? QEKF_FP32_BLOCK : 224; };
 #endif
 
-template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool MR, bool PF>
+template <typename T, bool BIAS, bool DIRECT, bool SYNTH, bool MR, bool PF, bool STATS>
 cudaError_t launch_run(const RunArgs<T> &a, unsigned grid, size_t smem, cudaStream_t stream);
 
 template <typename T, bool BIAS, bool PF>

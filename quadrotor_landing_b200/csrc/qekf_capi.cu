@@ -316,17 +316,24 @@ int run_typed(qekf_handle *h, const StreamView &in, int64_t k0, int64_t n_steps,
         // array belongs to filter d_perm[j], which is what keys its noise
         a.st.gid_perm = h->in_slot_order ? h->d_perm : nullptr;
         a.st.hist_synth = h->lazy_now ? 1 : 0;
-        if (h->stats_acc && truth && h->stats_stride > 0) {
-            a.stats.acc = h->stats_acc; a.stats.truth = truth;
-            a.stats.n_bins = h->stats_bins; a.stats.stride = h->stats_stride;
-            // two-sided 95% chi-square interval for n degrees of freedom
-            a.stats.chi2_lo = BIAS ? 6.262137795043251 : 2.7003894999803584;
-            a.stats.chi2_hi = BIAS ? 27.488392863442982 : 19.02276779864163;
-        }
+    }
+    // truth: the shared scenario truth [T+1][10] of a Monte-Carlo launch, or the per-filter truth of an explicit-stream
+    // launch (qekf_run_with_truth: [bin][16][N], based so that absolute bin indices work)
+    if (h->stats_acc && truth && h->stats_stride > 0) {
+        a.stats.acc = h->stats_acc;
+        if (ns) a.stats.truth = truth;
+        else { a.stats.truth_pf = truth; a.stats.ld_t = h->n; }
+        a.stats.n_bins = h->stats_bins; a.stats.stride = h->stats_stride;
+        // two-sided 95% chi-square interval for n degrees of freedom
+        a.stats.chi2_lo = BIAS ? 6.262137795043251 : 2.7003894999803584;
+        a.stats.chi2_hi = BIAS ? 27.488392863442982 : 19.02276779864163;
     }
     const bool mr = h->p.multirate_ekf != 0, pf = h->pf_on;
+    // explicit streams scored against per-filter truth run one thread per filter whatever the mapping says (the
+    // cooperative kernels accumulate statistics for Monte-Carlo launches only)
+    const bool coop_ok = ns != nullptr || a.stats.acc == nullptr;
     if constexpr (std::is_same<T, double>::value) {
-        if (!mr && h->lanes_per_filter == 2) {
+        if (!mr && h->lanes_per_filter == 2 && coop_ok) {
             // two role-specialised warps per 32 filters (ekf_duo.cuh)
             cudaError_t e;
             if (ns) e = pf ? launch_run_duo<BIAS, DIRECT, true, true>(a, h->duo_groups, h->stream)
@@ -337,7 +344,7 @@ int run_typed(qekf_handle *h, const StreamView &in, int64_t k0, int64_t n_steps,
             h->launches++;
             return QEKF_OK;
         }
-        if (!mr && h->lanes_per_filter == 3) {
+        if (!mr && h->lanes_per_filter == 3 && coop_ok) {
             // three lanes per filter (ekf_coop.cuh)
             cudaError_t e;
             if (ns) e = pf ? launch_run_coop<BIAS, DIRECT, true, true>(a, h->coop_groups, h->stream)
@@ -349,16 +356,17 @@ int run_typed(qekf_handle *h, const StreamView &in, int64_t k0, int64_t n_steps,
             return QEKF_OK;
         }
     }
-#define LAUNCH_(S, MR_, PF_) CUDA_TRY((launch_run<T, BIAS, DIRECT, S, MR_, PF_>(a, grid_of(h), smem_bytes(h), h->stream)))
-#define LAUNCH_S(S)                                                       \
+#define LAUNCH_(S, MR_, PF_, ST) CUDA_TRY((launch_run<T, BIAS, DIRECT, S, MR_, PF_, ST>(a, grid_of(h), smem_bytes(h), h->stream)))
+#define LAUNCH_S(S, ST)                                                   \
     do {                                                                  \
-        if (mr && pf) LAUNCH_(S, true, true);                             \
-        else if (mr) LAUNCH_(S, true, false);                             \
-        else if (pf) LAUNCH_(S, false, true);                             \
-        else LAUNCH_(S, false, false);                                    \
+        if (mr && pf) LAUNCH_(S, true, true, ST);                         \
+        else if (mr) LAUNCH_(S, true, false, ST);                         \
+        else if (pf) LAUNCH_(S, false, true, ST);                         \
+        else LAUNCH_(S, false, false, ST);                                \
     } while (0)
-    if (ns) LAUNCH_S(true);
-    else LAUNCH_S(false);
+    if (ns) LAUNCH_S(true, true);
+    else if (a.stats.acc) LAUNCH_S(false, true);     // explicit streams scored against per-filter truth
+    else LAUNCH_S(false, false);
 #undef LAUNCH_S
 #undef LAUNCH_
     h->launches++;
@@ -954,8 +962,14 @@ int qekf_filter_update(qekf_handle *h, double t_curr)
 
 int qekf_run(qekf_handle *h, const qekf_streams *s, int64_t k0, int64_t n_steps)
 {
+    return qekf_run_with_truth(h, s, nullptr, k0, n_steps);
+}
+
+int qekf_run_with_truth(qekf_handle *h, const qekf_streams *s, const double *truth, int64_t k0, int64_t n_steps)
+{
     if (h) hist_touch(h);
     if (!h || !s) return fail(QEKF_ERR_BAD_ARG, "NULL argument");
+    if (truth && !h->stats_acc) return fail(QEKF_ERR_NOT_INITIALIZED, "truth given but statistics are not configured");
     if (n_steps == 0) return QEKF_OK;
     if (k0 < 0 || n_steps < 0 || k0 + n_steps > s->T) return fail(QEKF_ERR_BAD_ARG, "tick range outside the stream");
     if (k0 + n_steps > 2147483647LL) return fail(QEKF_ERR_BAD_ARG, "tick indices are limited to 31 bits (as tag_step is)");
@@ -964,6 +978,14 @@ int qekf_run(qekf_handle *h, const qekf_streams *s, int64_t k0, int64_t n_steps)
         return fail(QEKF_ERR_BAD_ARG, "tag streams are NULL");
     CUDA_TRY(cudaSetDevice(h->device));
     const int64_t N = h->n, M = s->M, T = s->T;
+    // the bins sampled by this call: bin b is sampled after tick (b+1)*stride - 1, so [k0, k0+n_steps) holds the bins
+    // [k0/stride, (k0+n_steps)/stride), clipped to the configured ones.  None: a plain replay (nothing to score).
+    int64_t b_lo = 0, b_hi = 0;
+    if (truth) {
+        b_lo = std::min<int64_t>(k0 / h->stats_stride, h->stats_bins);
+        b_hi = std::min<int64_t>((k0 + n_steps) / h->stats_stride, h->stats_bins);
+        if (b_hi <= b_lo) truth = nullptr;
+    }
 
     // arrivals must be strictly increasing; the first one at or after k0 is where this launch starts
     std::vector<int32_t> steps_host;
@@ -987,14 +1009,17 @@ int qekf_run(qekf_handle *h, const qekf_streams *s, int64_t k0, int64_t n_steps)
         in.imu = s->imu; in.tag_step = s->tag_step; in.tag_pose = s->tag_pose;
         in.tag_stamp = s->tag_stamp; in.tag_valid = s->tag_valid;
     } else {
-        // host streams: stage the ticks of this call (and every arrival) into one device slab
+        // host streams: stage the ticks of this call (and every arrival), and the truth of the bins it samples, into one
+        // device slab
         const size_t imu_b = (size_t)n_steps * 6 * (size_t)N * 8;
         const size_t pose_b = (size_t)M * 7 * (size_t)N * 8;
         const size_t stamp_b = (size_t)M * 8, step_b = (size_t)M * 4;
         const size_t valid_b = s->tag_valid ? (size_t)M * (size_t)N : 0;
+        const size_t truth_b = truth ? (size_t)(b_hi - b_lo) * 16 * (size_t)N * 8 : 0;
         size_t o_imu = 0, o_pose = align_up(o_imu + imu_b, 256), o_stamp = align_up(o_pose + pose_b, 256);
         size_t o_step = align_up(o_stamp + stamp_b, 256), o_valid = align_up(o_step + step_b, 256);
-        size_t total = align_up(o_valid + valid_b, 256);
+        size_t o_truth = align_up(o_valid + valid_b, 256);
+        size_t total = align_up(o_truth + truth_b, 256);
         int rc = ensure_in(h, total);
         if (rc) return rc;
         char *d = (char *)h->d_in;
@@ -1011,9 +1036,15 @@ int qekf_run(qekf_handle *h, const qekf_streams *s, int64_t k0, int64_t n_steps)
         in.tag_stamp = (const double *)(d + o_stamp);
         in.tag_step = (const int32_t *)(d + o_step);
         in.tag_valid = valid_b ? (const uint8_t *)(d + o_valid) : nullptr;
+        if (truth_b) {
+            CUDA_TRY(cudaMemcpyAsync(d + o_truth, truth + (size_t)b_lo * 16 * (size_t)N, truth_b, cudaMemcpyHostToDevice,
+                                     h->stream));
+            // as the imu slab: the staged bins start at b_lo, bias the base pointer so absolute bin indices work
+            truth = (const double *)(d + o_truth) - (size_t)b_lo * 16 * (size_t)N;
+        }
     }
     (void)T;
-    return run_dispatch(h, in, k0, n_steps, m0);
+    return run_dispatch(h, in, k0, n_steps, m0, nullptr, truth);
 }
 
 // ---- accessors ---------------------------------------------------------------------------------------

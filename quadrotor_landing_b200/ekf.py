@@ -114,9 +114,10 @@ class BatchEKF:
         check(self._L.qekf_filter_update(self._h, float(t_curr)))
 
     # ---- batch replay ----
-    def run(self, k0, n_steps, imu, tag_step, tag_pose, tag_stamp, tag_valid=None, t_start=0.0):
+    def run(self, k0, n_steps, imu, tag_step, tag_pose, tag_stamp, tag_valid=None, t_start=0.0, truth=None):
         """Host (numpy) streams: imu [T][6][N], tag_step [M], tag_pose [M][7][N], tag_stamp [M],
-        tag_valid [M][N] or None."""
+        tag_valid [M][N] or None.  truth: [n_bins][16][N] per-filter true states (r v q_tv ab wb) after the sampling
+        tick of each statistics bin, or None; scores the replay into the statistics of stats_configure()."""
         imu = _f64(imu)
         T = imu.shape[0]
         assert imu.shape == (T, 6, self.N), imu.shape
@@ -137,19 +138,26 @@ class BatchEKF:
             s.tag_valid = tag_valid.ctypes.data
         s.t_start = float(t_start)
         s.on_device = 0
-        check(self._L.qekf_run(self._h, C.byref(s), int(k0), int(n_steps)))
+        tp = None
+        if truth is not None:
+            truth = _f64(truth)
+            assert truth.ndim == 3 and truth.shape[1:] == (16, self.N), truth.shape
+            tp = truth.ctypes.data
+        check(self._L.qekf_run_with_truth(self._h, C.byref(s), tp, int(k0), int(n_steps)))
         self.sync()   # the host buffers above must outlive the asynchronous copies
 
     def run_device(self, k0, n_steps, T, imu_ptr, M, tag_step_ptr, tag_pose_ptr, tag_stamp_ptr,
-                   tag_valid_ptr=None, t_start=0.0):
-        """Device-resident streams given as raw device pointers (e.g. torch tensors' data_ptr())."""
+                   tag_valid_ptr=None, t_start=0.0, truth_ptr=None):
+        """Device-resident streams given as raw device pointers (e.g. torch tensors' data_ptr()).  truth_ptr: device
+        pointer to the [n_bins][16][N] per-filter truth of run(), or None."""
         s = QekfStreams()
         s.T, s.imu, s.M = int(T), int(imu_ptr), int(M)
         s.tag_step, s.tag_pose, s.tag_stamp = tag_step_ptr, tag_pose_ptr, tag_stamp_ptr
         s.tag_valid = tag_valid_ptr
         s.t_start = float(t_start)
         s.on_device = 1
-        check(self._L.qekf_run(self._h, C.byref(s), int(k0), int(n_steps)))
+        tp = int(truth_ptr) if truth_ptr is not None else None
+        check(self._L.qekf_run_with_truth(self._h, C.byref(s), tp, int(k0), int(n_steps)))
 
     # ---- Monte-Carlo replay: shared clean scenario + in-kernel per-filter noise ----
     def _shared(self, scn, with_truth=True):

@@ -165,6 +165,32 @@ int qekf_latch_tag(qekf_handle *h, const double pos[3], const double quat_xyzw[4
 int qekf_tick(qekf_handle *h, const double accel[3], const double gyro[3], int tag_mode, const double tag_pos[3],
               const double tag_quat_xyzw[4], double tag_stamp, double t_curr, int n_out, double *records);
 
+/* One timer tick of every filter of the handle with per-filter inputs, all pointers DEVICE memory, asynchronous on the
+ * handle's stream, no host synchronisation, no allocation: legal inside CUDA stream capture.  For estimator-in-the-loop
+ * simulation, where the next IMU sample depends on the estimate and no input stream exists ahead of time.
+ * Per filter i, the node's tick sequence (relative_pose_EKF_node.cpp:144-182) in the order the batch replay uses:
+ *   if arrived[i] != 0: AprilTagSubCallback with the filter's own pose and stamp (node.cpp:153-176: latch,
+ *                       measurement_ready, first-detection initialize_state);
+ *   IMUSubCallback with imu[:, i] (node.cpp:144-151), then filter_update(t_curr) (node.cpp:178-182);
+ *   the requested outputs, converted to double for QEKF_FP32 handles.
+ * Every output pointer may be NULL (not written).  All arrays are [component][N], N = qekf_num_filters.
+ * Every variant is served (precision, est_bias, direct_orien_method, single rate / fixed / dynamic delay, per-filter
+ * parameters); one thread per filter whatever qekf_set_mapping says.  Like qekf_tick, a step counts as a touch of the
+ * delayed-fusion histories: a later qekf_run_monte_carlo replays them from the ring.  QEKF_ERR_BAD_ARG for a NULL h,
+ * io or imu, for arrived without tag, and for pointers the driver reports as unregistered host memory or as memory of
+ * another device. */
+typedef struct qekf_step_io {
+    const double  *imu;        /* [6][N]  accel xyz, gyro xyz: IMUSubCallback of each filter                       */
+    const uint8_t *arrived;    /* [N] or NULL: nonzero = a detection arrived since the last tick (AprilTagSubCallback:
+                                  latch, measurement_ready, first-detection initialize_state)                        */
+    const double  *tag;        /* [8][N]  r_c_tc xyz, q_ct xyzw, capture stamp; read only where arrived[i] != 0      */
+    double  *x_out;            /* [16][N]   or NULL: layout of the state accessor (r v q_xyzw ab wb)                */
+    double  *cov_out;          /* [n(n+1)/2][N] or NULL: upper triangle of cov_pert, row by row (a <= b)            */
+    double  *aux_out;          /* [11][N]   or NULL: layout of the aux accessor                                     */
+    int32_t *flags_out;        /* [6][N]    or NULL: layout of the flags accessor                                   */
+} qekf_step_io;
+int qekf_step(qekf_handle *h, double t_curr, const qekf_step_io *io);
+
 /* ---- batch replay: filter_update iterated n_steps times inside one kernel launch -------------- */
 
 /* Explicit per-filter input streams.  Tick k (absolute index) runs at t_curr = t_start + k/update_freq.

@@ -104,6 +104,19 @@ class QekfNoiseSpec(C.Structure):
     ]
 
 
+class QekfStepIO(C.Structure):
+    """qekf_step_io: device pointers of one qekf_step call (NULL = not given)."""
+    _fields_ = [
+        ("imu", C.c_void_p),
+        ("arrived", C.c_void_p),
+        ("tag", C.c_void_p),
+        ("x_out", C.c_void_p),
+        ("cov_out", C.c_void_p),
+        ("aux_out", C.c_void_p),
+        ("flags_out", C.c_void_p),
+    ]
+
+
 class QekfSharedStreams(C.Structure):
     _fields_ = [
         ("T", C.c_int64),
@@ -126,7 +139,7 @@ EXPORTS = [
     "qekf_default_params", "qekf_create", "qekf_destroy", "qekf_set_params", "qekf_get_params",
     "qekf_set_filter_params", "qekf_last_error_string", "qekf_num_states", "qekf_num_filters",
     "qekf_set_mapping", "qekf_set_stream", "qekf_sync", "qekf_set_imu", "qekf_set_tag", "qekf_initialize_state",
-    "qekf_filter_update", "qekf_latch_tag", "qekf_tick", "qekf_run", "qekf_run_with_truth", "qekf_get_state", "qekf_get_cov", "qekf_get_aux", "qekf_get_flags",
+    "qekf_filter_update", "qekf_latch_tag", "qekf_tick", "qekf_step", "qekf_run", "qekf_run_with_truth", "qekf_get_state", "qekf_get_cov", "qekf_get_aux", "qekf_get_flags",
     "qekf_set_state", "qekf_prediction_step", "qekf_correction_step",
     "qekf_scenario_default", "qekf_scenario_sizes", "qekf_scenario_generate",
     "qekf_noise_default", "qekf_run_monte_carlo", "qekf_synthesize_streams", "qekf_stats_configure",
@@ -168,6 +181,7 @@ def lib() -> C.CDLL:
     L.qekf_filter_update.argtypes = [vp, C.c_double]
     L.qekf_latch_tag.argtypes = [vp, dp, dp, C.c_double]
     L.qekf_tick.argtypes = [vp, dp, dp, C.c_int, dp, dp, C.c_double, C.c_double, C.c_int, dp]
+    L.qekf_step.argtypes = [vp, C.c_double, C.POINTER(QekfStepIO)]
     L.qekf_run.argtypes = [vp, C.POINTER(QekfStreams), C.c_int64, C.c_int64]
     L.qekf_run_with_truth.argtypes = [vp, C.POINTER(QekfStreams), vp, C.c_int64, C.c_int64]
     L.qekf_get_state.argtypes = [vp, C.c_int64, C.c_int64, dp]

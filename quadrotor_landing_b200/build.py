@@ -39,6 +39,8 @@ def _units():
                 for m in (0, 1):
                     units.append(("inst_run_%s_b%d_d%d_m%d" % (t, b, d, m), "inst_run.cu",
                                   ["-DQ_T=%s" % t, "-DQ_BIAS=%d" % b, "-DQ_DIRECT=%d" % d, "-DQ_MR=%d" % m]))
+                    units.append(("inst_step_%s_b%d_d%d_m%d" % (t, b, d, m), "inst_step.cu",
+                                  ["-DQ_T=%s" % t, "-DQ_BIAS=%d" % b, "-DQ_DIRECT=%d" % d, "-DQ_MR=%d" % m]))
     return units
 
 
@@ -46,7 +48,8 @@ def is_stale() -> bool:
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    srcs = HEADERS + COOP_HEADERS + ["qekf_capi.cu", "inst_misc.cu", "inst_run.cu", "inst_coop.cu", "inst_duo.cu"]
+    srcs = HEADERS + COOP_HEADERS + ["qekf_capi.cu", "inst_misc.cu", "inst_run.cu", "inst_step.cu", "inst_coop.cu",
+                                      "inst_duo.cu"]
     return any(os.path.getmtime(os.path.join(CSRC, f)) > t for f in srcs)
 
 

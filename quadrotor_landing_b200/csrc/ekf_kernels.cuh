@@ -1366,14 +1366,15 @@ QEKF_FN void rebase_history(const DeviceState<T> &st, int64_t i, const Nominal<T
 // AprilTagSubCallback for filter i with pose8 = (position, orientation xyzw, stamp)  (node.cpp:153-176):
 // latch the pose, raise measurement_ready (unless raise_ready = 0: the latch only, what a forced initialize_state
 // of the facade needs), initialise on the first detection; force_init: initialize_state from the latched members.
+// Component cc of the pose is pose8[cc * ps]: 1 for one pose shared by all filters, N for a [8][N] per-filter array.
 template <typename T, bool BIAS, bool PF, class PS>
 QEKF_FN void deliver_one(const DeviceState<T> &st, const Consts<T> &c, const double *pose8, int force_init, int reinit_bias,
-                         int raise_ready, PS &P, int64_t i)
+                         int raise_ready, PS &P, int64_t i, int64_t ps = 1)
 {
     int32_t flags = st.flags[i];
     if (!force_init) {
 #pragma unroll
-        for (int cc = 0; cc < PEND_DIM; ++cc) st.pend[cc * st.ld + i] = pose8[cc];
+        for (int cc = 0; cc < PEND_DIM; ++cc) st.pend[cc * st.ld + i] = pose8[cc * ps];
         if (raise_ready) flags |= FLAG_READY;
     }
     if (force_init || (raise_ready && !(flags & FLAG_INIT))) {
@@ -1455,6 +1456,270 @@ __global__ void __launch_bounds__(TICK_BLOCK) tick_kernel(const __grid_constant_
             }
             r[e] = v;
         }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// per-tick step with per-filter device inputs and outputs (qekf_step: estimator-in-the-loop simulation)
+// ------------------------------------------------------------------------------------------------
+// One launch = one timer tick of every filter: the tag callback where a detection arrived, then the IMU sample and
+// filter_update(t_curr), then the members the caller asked for.  Inputs and outputs are [c][N] device arrays.
+template <typename T> struct StepArgs {
+    DeviceState<T> st;
+    Consts<T> c;
+    double t_curr;
+    const double *imu;        // [6][n]
+    const uint8_t *arrived;   // [n] or nullptr
+    const double *tag;        // [8][n]
+    double *x_out, *cov_out, *aux_out;   // [16][n], [NP][n], [11][n] or nullptr
+    int32_t *flags_out;       // [6][n] or nullptr
+};
+
+// What a step leaves in registers for the outputs (the covariance stays in the caller's PS).
+template <typename T> struct StepOut {
+    Nominal<T> s;
+    T accel[3];
+    int32_t flags, upds, hlen;
+    uint32_t n_pred, n_corr;
+};
+
+// x and P of filter i from the [16][ld] / [NP][ld] arrays x, Pg.  On the device the covariance goes straight to shared
+// memory through cp.async: all NP loads of a lane are in flight at once and hold no registers (this kernel is bound by
+// memory, and the per-lane loop of load_filter keeps only a few loads in flight).
+template <typename T, class PS>
+QEKF_FN void step_load(const T *x, const T *Pg, int64_t ld, int64_t i, Nominal<T> &s, PS &P)
+{
+    constexpr int N = PS::n;
+    constexpr int NP = N * (N + 1) / 2;
+#ifdef __CUDA_ARCH__
+#pragma unroll 8
+    for (int e = 0; e < NP; ++e) {
+        const uint32_t dst = (uint32_t)__cvta_generic_to_shared(&P.el(e));
+        if (sizeof(T) == 8) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst), "l"(Pg + e * ld + i) : "memory");
+        else asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(Pg + e * ld + i) : "memory");
+    }
+#endif
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        s.r[k] = x[(0 + k) * ld + i];
+        s.v[k] = x[(3 + k) * ld + i];
+        s.ab[k] = x[(10 + k) * ld + i];
+        s.wb[k] = x[(13 + k) * ld + i];
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) s.q[k] = x[(6 + k) * ld + i];
+#ifdef __CUDA_ARCH__
+    asm volatile("cp.async.wait_all;" ::: "memory");   // (the copies of this lane are visible to this lane)
+#else
+    for (int e = 0; e < NP; ++e) P.el(e) = Pg[e * ld + i];
+#endif
+}
+
+// One tick of filter i (AprilTagSubCallback already applied) with IMU sample u_in[cc * us]: filter_update(t_curr)
+// (cpp:127-303) as run_filter / run_filter_mr sequence it for one tick.  On return P holds the head covariance and o the
+// head state.  Host-callable (tests/host_core/host_step.cu).
+//
+// Delayed fusion keeps the HEAD current instead of materialising it from the checkpoint: after any launch st.x / st.P
+// hold the head and xc / Pc / ring / nh / hpos / hlen the history (ekf_kernels.cuh, run_filter_mr), so
+//   - a tick that fuses nothing advances the head by one prediction_step and pushes its input into the ring; the
+//     checkpoint is only touched when the ring is full (catch-up to entry size-D, as the replay does);
+//   - a tick that fuses a measurement does what the lazy loop does: advance the checkpoint to the corrected entry,
+//     correct there, store the new checkpoint, replay the ring to the head.
+// Every entry is the same chain of prediction_steps through advance_call as in the replay, so the head is bit-identical
+// to the one the replay materialises, and the state left behind is what every other entry point expects.  Per tick:
+// 1 prediction, plus nh + ~1 on the ticks that fuse (~2 + d / upd_per_meas per tick on average, d = step delay).
+// The head and the checkpoint are never needed at the same time: one covariance buffer (NP values per lane) serves both.
+template <typename T, bool BIAS, bool DIRECT, bool MR, bool PF, class PS>
+QEKF_FN void step_filter(const DeviceState<T> &st, const Consts<T> &c, int64_t i, double t_curr, const double *u_in,
+                         int64_t us, PS &P, StepOut<T> &o)
+{
+    const typename ParSel<T, PF>::type par = ParSel<T, PF>::make(c, st, i);
+    int32_t flags = st.flags[i], upds = st.upds[i];
+    T accel[3];
+#pragma unroll
+    for (int cc = 0; cc < 3; ++cc) accel[cc] = st.aux[cc * st.ld + i];
+    T u[6];
+#pragma unroll
+    for (int cc = 0; cc < 6; ++cc) u[cc] = (T)u_in[cc * us];
+    const bool init = (flags & FLAG_INIT) != 0;
+    // cpp:147: the measurement gate; consume the latched measurement, corner-margin gate (cpp:150-186)
+    const bool want = init && (flags & FLAG_READY) && (!c.limit_measurement_freq || (upds + 1) >= c.upd_per_meas);
+    bool perform = false;
+    T tag[7];
+    double stamp = 0;
+    if (want) {
+        double tg[7];       // the gate decides on the double pose
+#pragma unroll
+        for (int cc = 0; cc < 7; ++cc) tg[cc] = st.pend[cc * st.ld + i];
+        stamp = st.pend[7 * st.ld + i];
+#pragma unroll
+        for (int cc = 0; cc < 7; ++cc) tag[cc] = (T)tg[cc];
+        flags &= ~FLAG_READY;
+        perform = c.corner_margin_enbl ? corner_gate<T>(tg, c) : true;
+    }
+    Nominal<T> s;
+    uint32_t n_pred = 0, n_corr = 0;
+    int32_t hl = init ? 1 : 0;
+    if (!MR) {
+        step_load<T>(st.x, st.P, st.ld, i, s, P);
+        if (init) {
+            prediction_step<T, BIAS>(s, P, u, par, accel);
+            ++n_pred;
+        }
+        if (perform) {
+            ++n_corr;
+            Observation<T> obs;
+            correction_step<T, BIAS, DIRECT>(s, P, tag, par, obs);
+#pragma unroll
+            for (int cc = 0; cc < 3; ++cc) st.aux[(3 + cc) * st.ld + i] = obs.r_t_vt_obs[cc];
+#pragma unroll
+            for (int cc = 0; cc < 4; ++cc) st.aux[(6 + cc) * st.ld + i] = obs.q_tv_obs[cc];
+        }
+        if (init) store_filter<T>(st, i, s, P);
+    } else {
+        const int32_t L = st.ring_len, Dm1 = st.dmax_m1;
+        T *ring_i = st.ring + i;
+        int32_t nh = 0, hpos = 0;
+        if (init) { nh = st.nh[i]; hpos = st.hpos[i]; hl = st.hlen[i]; }
+        // the input of this tick joins the history (cpp:240-257): ring slot after the head
+        auto push = [&]() {
+            hpos = (hpos + 1 == L) ? 0 : hpos + 1;
+#pragma unroll
+            for (int cc = 0; cc < 6; ++cc) ring_i[((int64_t)hpos * 6 + cc) * st.ld] = u[cc];
+            ++nh; ++hl;
+        };
+        auto oldest = [&]() { const int32_t f = hpos - nh + 1; return f < 0 ? f + L : f; };
+        if (!init) {
+            step_load<T>(st.x, st.P, st.ld, i, s, P);      // (read only for the outputs)
+        } else if (perform) {
+            // cpp:199-201
+            const double delay = c.dynamic_meas_delay ? fmin(t_curr - stamp + par.dyn_offset(), c.meas_delay_max)
+                                                      : par.meas_delay();
+            int32_t step = (int32_t)(delay / c.dT_nom + 0.5);
+            if (step < 1) step = 1;
+            int32_t ind = hl - step;
+            if (ind < 0) ind = 0;
+            int32_t n_adv = ind - (hl - 1 - nh);          // >= 0 by the ring invariant
+            if (n_adv < 0) n_adv = 0;
+            st.aux[10 * st.ld + i] = (T)delay;            // measurement_delay_curr
+            step_load<T>(st.xc, st.Pc, st.ld, i, s, P);
+            T scratch[3] = { T(0), T(0), T(0) };
+            advance_call<T, BIAS>(&s, P, par, ring_i, st.ld, L, oldest(), n_adv, scratch);
+            nh -= n_adv;
+            ++n_corr;
+            Observation<T> obs;
+            correction_call<T, BIAS, DIRECT>(&s, P, tag, par, &obs);
+#pragma unroll
+            for (int cc = 0; cc < 3; ++cc) st.aux[(3 + cc) * st.ld + i] = obs.r_t_vt_obs[cc];
+#pragma unroll
+            for (int cc = 0; cc < 4; ++cc) st.aux[(6 + cc) * st.ld + i] = obs.q_tv_obs[cc];
+            hl = nh + 1;                                  // history before the corrected entry is erased (cpp:214-219)
+            store_checkpoint<T>(st, i, s, P);
+            push();
+            advance_call<T, BIAS>(&s, P, par, ring_i, st.ld, L, oldest(), nh, accel);   // the re-propagation (cpp:222-226)
+            n_pred += (uint32_t)(n_adv + nh);
+        } else {
+            if (nh >= L - 1) {
+                // the ring is full: catch the checkpoint up to entry size-D (never past it, see run_filter_mr)
+                const int32_t n_c = nh - Dm1;
+                step_load<T>(st.xc, st.Pc, st.ld, i, s, P);
+                T scratch[3] = { T(0), T(0), T(0) };
+                advance_call<T, BIAS>(&s, P, par, ring_i, st.ld, L, oldest(), n_c, scratch);
+                store_checkpoint<T>(st, i, s, P);
+                nh -= n_c;
+                n_pred += (uint32_t)n_c;
+            }
+            step_load<T>(st.x, st.P, st.ld, i, s, P);
+            push();
+            advance_call<T, BIAS>(&s, P, par, ring_i, st.ld, L, hpos, 1, accel);        // the head prediction
+            ++n_pred;
+        }
+        if (init) {
+            store_filter<T>(st, i, s, P);
+            st.nh[i] = nh; st.hpos[i] = hpos; st.hlen[i] = hl;
+        }
+    }
+    if (init) {
+        if (perform) { upds = 0; flags |= FLAG_CORRECTED; }
+        else { upds += 1; flags &= ~FLAG_CORRECTED; }
+        flags |= FLAG_ACTIVE;
+    }
+    st.flags[i] = flags;
+    st.upds[i] = upds;
+#pragma unroll
+    for (int cc = 0; cc < 3; ++cc) st.aux[cc * st.ld + i] = accel[cc];
+    o.s = s;
+#pragma unroll
+    for (int cc = 0; cc < 3; ++cc) o.accel[cc] = accel[cc];
+    o.flags = flags; o.upds = upds; o.hlen = hl;
+    o.n_pred = n_pred; o.n_corr = n_corr;
+}
+
+// The requested outputs of filter i, [c][n] rows: the state and flags from registers, the covariance from the lane's
+// shared-memory column.  Rows 3..10 of aux are only rewritten by a correction and are read back from st.aux.
+template <typename T, class PS>
+QEKF_FN void step_outputs(const StepArgs<T> &a, int64_t i, const StepOut<T> &o, const PS &P)
+{
+    constexpr int N = PS::n;
+    constexpr int NP = N * (N + 1) / 2;
+    const int64_t n = a.st.n;
+    if (a.x_out) {
+        double *x = a.x_out + i;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            x[(0 + k) * n] = (double)o.s.r[k];
+            x[(3 + k) * n] = (double)o.s.v[k];
+            x[(10 + k) * n] = (double)o.s.ab[k];
+            x[(13 + k) * n] = (double)o.s.wb[k];
+        }
+#pragma unroll
+        for (int k = 0; k < 4; ++k) x[(6 + k) * n] = (double)o.s.q[k];
+    }
+    if (a.cov_out) {
+#pragma unroll 8
+        for (int e = 0; e < NP; ++e) a.cov_out[e * n + i] = (double)P.el(e);
+    }
+    if (a.aux_out) {
+#pragma unroll
+        for (int cc = 0; cc < 3; ++cc) a.aux_out[cc * n + i] = (double)o.accel[cc];
+#pragma unroll
+        for (int cc = 3; cc < AUX_DIM; ++cc) a.aux_out[cc * n + i] = (double)a.st.aux[cc * a.st.ld + i];
+    }
+    if (a.flags_out) {
+        int32_t *f = a.flags_out + i;
+        f[0 * n] = (o.flags & FLAG_INIT) ? 1 : 0;
+        f[1 * n] = (o.flags & FLAG_READY) ? 1 : 0;
+        f[2 * n] = (o.flags & FLAG_CORRECTED) ? 1 : 0;
+        f[3 * n] = (o.flags & FLAG_ACTIVE) ? 1 : 0;
+        f[4 * n] = o.upds;
+        f[5 * n] = o.hlen;     // x_hist.size(): 0 before initialisation, 1 for single-rate filters
+    }
+}
+
+// qekf_step: one thread per filter, covariance staged in shared memory (element-major, as run_kernel).  Memory-bound:
+// a tick loads and stores the whole filter state.  BLOCK: see launch_step (inst_step.cu).
+template <typename T, bool BIAS, bool DIRECT, bool MR, bool PF, int BLOCK>
+__global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ StepArgs<T> a)
+{
+    constexpr int N = BIAS ? 15 : 9;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    T *sm = reinterpret_cast<T *>(smem_raw);
+    const int64_t i = (int64_t)blockIdx.x * BLOCK + threadIdx.x;
+    const bool live = i < a.st.n;
+    PShared<T, N, BLOCK> P{ sm + threadIdx.x };
+    StepOut<T> o;
+    o.n_pred = 0; o.n_corr = 0;
+    if (live) {
+        if (a.arrived && a.arrived[i]) deliver_one<T, BIAS, PF>(a.st, a.c, a.tag + i, 0, 0, 1, P, i, a.st.n);
+        step_filter<T, BIAS, DIRECT, MR, PF>(a.st, a.c, i, a.t_curr, a.imu + i, a.st.n, P, o);
+        step_outputs<T>(a, i, o, P);
+    }
+    // the work counters: one atomic per warp (all lanes get here: BLOCK is a multiple of 32)
+    const unsigned full = 0xffffffffu;
+    const unsigned np = __reduce_add_sync(full, o.n_pred), nc = __reduce_add_sync(full, o.n_corr);
+    if ((threadIdx.x & 31) == 0 && a.st.counts) {
+        if (np) atomicAdd(a.st.counts + 0, (unsigned long long)np);
+        if (nc) atomicAdd(a.st.counts + 1, (unsigned long long)nc);
     }
 }
 

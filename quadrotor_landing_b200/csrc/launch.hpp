@@ -32,6 +32,17 @@ cudaError_t launch_deliver(const DeviceState<T> &st, const Consts<T> &c, const d
 template <typename T, bool BIAS, bool DIRECT, bool MR>
 cudaError_t launch_tick(const RunArgs<T> &a, const double *pose8, int tag_mode, double *out, int n_out, cudaStream_t stream);
 
+// qekf_step (step_kernel, inst_step.cu).  block: CTA size, one of STEP_BLOCKS.  prep_step sets the kernel's dynamic
+// shared-memory attribute; the handle calls it where it is created or re-parameterised, so that launch_step issues
+// nothing but the launch (legal inside stream capture).
+// Measured on a B200 (1,000 W) with tools/probe_step.py, N = 65,536 .. 1,048,576: FP64 is fastest at 32 threads (up to 12 %
+// ahead of 128: more CTAs fit the shared memory the covariance takes), FP32 at 128 (1-4 % ahead of 32).
+constexpr int STEP_BLOCKS[3] = { 32, 64, 128 };
+constexpr int step_block_default(bool fp64) { return fp64 ? 32 : 128; }
+template <typename T, bool BIAS, bool DIRECT, bool MR, bool PF> cudaError_t prep_step(int block);
+template <typename T, bool BIAS, bool DIRECT, bool MR, bool PF>
+cudaError_t launch_step(const StepArgs<T> &a, int block, cudaStream_t stream);
+
 template <typename T, bool BIAS, bool PF>
 cudaError_t launch_predict(const DeviceState<T> &st, const Consts<T> &c, const double *u, unsigned grid, size_t smem,
                            cudaStream_t stream);

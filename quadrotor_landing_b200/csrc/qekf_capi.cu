@@ -111,6 +111,8 @@ struct qekf_handle {
     // warps per 32 filters (ekf_duo.cuh), 3 = three lanes per filter (ekf_coop.cuh), 1 = one thread per filter
     int lanes_per_filter = 1;
     int coop_groups = COOP_GROUPS_DEFAULT, duo_groups = DUO_GROUPS_DEFAULT;
+    // CTA size of the per-tick step kernel (qekf_step, launch.hpp); QEKF_STEP_BLOCK overrides it (A/B runs)
+    int step_block = 32;
 };
 
 namespace {
@@ -576,6 +578,62 @@ int tick_typed(qekf_handle *h, int tag_mode, double t_curr, int n_out)
     return QEKF_OK;
 }
 
+template <typename T, bool BIAS, bool DIRECT>
+int step_typed(qekf_handle *h, double t_curr, const qekf_step_io *io)
+{
+    StepArgs<T> a;
+    std::memset(&a, 0, sizeof a);
+    a.st = dstate<T>(h);
+    a.c = make_consts<T>(h->p);
+    a.t_curr = t_curr;
+    a.imu = io->imu; a.arrived = io->arrived; a.tag = io->tag;
+    a.x_out = io->x_out; a.cov_out = io->cov_out; a.aux_out = io->aux_out; a.flags_out = io->flags_out;
+    const bool mr = h->p.multirate_ekf != 0, pf = h->pf_on;
+#define LAUNCH_STEP(MR_, PF_) CUDA_TRY((launch_step<T, BIAS, DIRECT, MR_, PF_>(a, h->step_block, h->stream)))
+    if (mr && pf) LAUNCH_STEP(true, true);
+    else if (mr) LAUNCH_STEP(true, false);
+    else if (pf) LAUNCH_STEP(false, true);
+    else LAUNCH_STEP(false, false);
+#undef LAUNCH_STEP
+    h->launches++;
+    return QEKF_OK;
+}
+
+// the step kernels' launch attributes for the current parameters and precision, set here rather than at the launch, so
+// that qekf_step issues nothing but the kernel (it may be captured into a CUDA graph); called wherever the handle is
+// created or changes shape
+int prep_step_kernels(qekf_handle *h)
+{
+#define PREP_ONE(T_, B_, D_, MR_, PF_) CUDA_TRY((prep_step<T_, B_, D_, MR_, PF_>(h->step_block)))
+#define PREP_T(T_, B_, D_)                                                                                             \
+    do {                                                                                                               \
+        PREP_ONE(T_, B_, D_, false, false); PREP_ONE(T_, B_, D_, false, true);                                         \
+        PREP_ONE(T_, B_, D_, true, false); PREP_ONE(T_, B_, D_, true, true);                                           \
+    } while (0)
+    QEKF_DISPATCH(h, PREP_T);
+#undef PREP_T
+#undef PREP_ONE
+    return QEKF_OK;
+}
+
+// a pointer the step kernel may dereference: device memory of the handle's device, managed, or registered / pinned host
+// memory (cudaPointerGetAttributes queries the driver's tables only: it enqueues nothing and is legal during capture)
+int check_step_ptr(const qekf_handle *h, const void *p, const char *what)
+{
+    if (!p) return QEKF_OK;
+    cudaPointerAttributes at;
+    cudaError_t e = cudaPointerGetAttributes(&at, p);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(QEKF_ERR_BAD_ARG, std::string("qekf_step: cannot query ") + what);
+    }
+    if (at.type == cudaMemoryTypeUnregistered)
+        return fail(QEKF_ERR_BAD_ARG, std::string("qekf_step: ") + what + " is unregistered host memory (it must be device memory)");
+    if (at.type == cudaMemoryTypeDevice && at.device != h->device)
+        return fail(QEKF_ERR_BAD_ARG, std::string("qekf_step: ") + what + " lives on another device");
+    return QEKF_OK;
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
@@ -664,6 +722,7 @@ int qekf_create(const qekf_params *p, int64_t n_filters, int device, int precisi
     qekf_handle *h = new (std::nothrow) qekf_handle;
     if (!h) return fail(QEKF_ERR_ALLOC, "out of host memory");
     h->p = *p; h->precision = precision; h->device = device;
+    h->step_block = step_block_default(precision == QEKF_FP64);
     {   // environment overrides of the default mapping (profiling / A-B runs): QEKF_LANES=1|3, QEKF_COOP_GROUPS=n
         const char *e = getenv("QEKF_LANES");
         if (e && atoi(e) >= 1 && atoi(e) <= 3) h->lanes_per_filter = atoi(e);
@@ -677,6 +736,8 @@ int qekf_create(const qekf_params *p, int64_t n_filters, int device, int precisi
         if (e && atoll(e) > 0) h->perm_min_steps = atoll(e);
         e = getenv("QEKF_DUO_GROUPS");
         if (e && duo_groups_available(atoi(e), p->est_bias && p->direct_orien_method)) h->duo_groups = atoi(e);
+        e = getenv("QEKF_STEP_BLOCK");
+        if (e) for (int b : STEP_BLOCKS) if (atoi(e) == b) h->step_block = b;
     }
     h->n = n_filters; h->ld = (n_filters + 31) / 32 * 32;
     if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) {
@@ -686,6 +747,7 @@ int qekf_create(const qekf_params *p, int64_t n_filters, int device, int precisi
     h->own_stream = true;
     rc = alloc_state(h);
     if (!rc) rc = reset_cov(h, true);
+    if (!rc) rc = prep_step_kernels(h);
     if (rc) { free_state(h); cudaStreamDestroy(h->stream); delete h; return rc; }
     *out = h;
     return QEKF_OK;
@@ -717,6 +779,8 @@ int qekf_set_params(qekf_handle *h, const qekf_params *p)
     CUDA_TRY(cudaSetDevice(h->device));
     const bool shape_change = (p->est_bias != 0) != (h->p.est_bias != 0);
     h->p = *p;
+    rc = prep_step_kernels(h);     // (est_bias, direct_orien_method and multirate_ekf pick the step kernel)
+    if (rc) return rc;
     if (shape_change) {
         CUDA_TRY(cudaStreamSynchronize(h->stream));
         free_state(h);
@@ -940,6 +1004,25 @@ int qekf_tick(qekf_handle *h, const double accel[3], const double gyro[3], int t
     CUDA_TRY(cudaStreamSynchronize(h->stream));
     if (n_out > 0) std::memcpy(records, h->tick_out, (size_t)n_out * TICK_REC * sizeof(double));
     return QEKF_OK;
+}
+
+int qekf_step(qekf_handle *h, double t_curr, const qekf_step_io *io)
+{
+    if (h) hist_touch(h);
+    if (!h || !io || !io->imu) return fail(QEKF_ERR_BAD_ARG, "qekf_step: NULL handle, io or imu");
+    if (io->arrived && !io->tag) return fail(QEKF_ERR_BAD_ARG, "qekf_step: arrived given without tag");
+    CUDA_TRY(cudaSetDevice(h->device));
+    const void *ptrs[7] = { io->imu, io->arrived, io->tag, io->x_out, io->cov_out, io->aux_out, io->flags_out };
+    const char *names[7] = { "imu", "arrived", "tag", "x_out", "cov_out", "aux_out", "flags_out" };
+    for (int k = 0; k < 7; ++k) {
+        int rc = check_step_ptr(h, ptrs[k], names[k]);
+        if (rc) return rc;
+    }
+    int rc = QEKF_OK;
+#define CALL_STEP(T, B, D) rc = step_typed<T, B, D>(h, t_curr, io)
+    QEKF_DISPATCH(h, CALL_STEP);
+#undef CALL_STEP
+    return rc;
 }
 
 int qekf_filter_update(qekf_handle *h, double t_curr)

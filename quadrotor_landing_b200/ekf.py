@@ -159,6 +159,51 @@ class BatchEKF:
         tp = int(truth_ptr) if truth_ptr is not None else None
         check(self._L.qekf_run_with_truth(self._h, C.byref(s), tp, int(k0), int(n_steps)))
 
+    # ---- per-tick step with device-resident per-filter inputs and outputs (closed-loop simulation) ----
+    def step(self, t_curr, imu, tag=None, arrived=None, x=None, cov=None, aux=None, flags=None):
+        """One timer tick of every filter (qekf_step): for filter i, the tag callback with tag[:, i] where arrived[i] is
+        nonzero, then the IMU sample imu[:, i] and filter_update(t_curr).  All arguments are contiguous torch CUDA tensors
+        on this handle's device: imu [6][N] float64; tag [8][N] float64 (r_c_tc xyz, q_ct xyzw, capture stamp); arrived
+        [N] uint8 or bool.  Outputs, written where given and never allocated here: x [16][N], cov [n(n+1)/2][N] (upper
+        triangle of cov_pert, row by row), aux [11][N] float64, flags [6][N] int32 -- the accessors' layouts.  Returns
+        (x, cov, aux, flags).
+
+        Asynchronous on the handle's stream, with no host synchronisation, so it can be captured into a CUDA graph.  To
+        order it with torch work, run it on torch's stream: set_stream(torch.cuda.current_stream().cuda_stream)."""
+        import torch
+        dev = torch.device("cuda", self._device)
+        N = self.N
+
+        def ptr(t, name, rows, dtypes):
+            if t is None:
+                return None
+            if not isinstance(t, torch.Tensor) or t.device != dev:
+                raise ValueError("%s must be a torch tensor on %s" % (name, dev))
+            if t.dtype not in dtypes:
+                raise ValueError("%s must be %s, not %s" % (name, " or ".join(str(d) for d in dtypes), t.dtype))
+            shape = (N,) if rows is None else (rows, N)
+            if tuple(t.shape) != shape:
+                raise ValueError("%s must have shape %s, not %s" % (name, shape, tuple(t.shape)))
+            if not t.is_contiguous():
+                raise ValueError("%s must be contiguous" % name)
+            return t.data_ptr()
+
+        if imu is None:
+            raise ValueError("imu is required")
+        if arrived is not None and tag is None:
+            raise ValueError("arrived given without tag")
+        f64, n = (torch.float64,), self.n
+        io = nat.QekfStepIO()
+        io.imu = ptr(imu, "imu", 6, f64)
+        io.tag = ptr(tag, "tag", 8, f64)
+        io.arrived = ptr(arrived, "arrived", None, (torch.uint8, torch.bool))
+        io.x_out = ptr(x, "x", 16, f64)
+        io.cov_out = ptr(cov, "cov", n * (n + 1) // 2, f64)
+        io.aux_out = ptr(aux, "aux", 11, f64)
+        io.flags_out = ptr(flags, "flags", 6, (torch.int32,))
+        check(self._L.qekf_step(self._h, float(t_curr), C.byref(io)))
+        return x, cov, aux, flags
+
     # ---- Monte-Carlo replay: shared clean scenario + in-kernel per-filter noise ----
     def _shared(self, scn, with_truth=True):
         """scn: quadrotor_landing_b200.scenario.Scenario (host numpy arrays).  Returns the C struct and the
